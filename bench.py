@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # our CUDA path (one process per GPU under torchrun)
     python bench.py --impl reference --gpus N --steps K ...  # the reference's CPU arithmetic (oracle port) on the host cores
+    python bench.py ... --dump-outputs DIR                   # also write what the last timed step computed as DIR/<name>.npy
 
 One JSON line on stdout (rank 0).  A "step" is one pass of the hot path over one batch of synthetic input:
   * headline workload (BASELINE config 4, the one the target metric is quoted on): fused per-object frustum cull +
@@ -38,6 +39,7 @@ ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
 from rend3_b200.backend import CAMERA_VIEWPORT, CB_BAKE, CB_CULL  # noqa: E402
+from rend3_b200.layouts import OBJECT_MATRICES_DTYPE  # noqa: E402
 from rend3_b200.routines import BaseRenderGraph, BaseRenderGraphSettings, per_camera_header  # noqa: E402
 from rend3_b200.scenes import cloud_camera, cube_field_scene, object_cloud_records  # noqa: E402
 
@@ -83,6 +85,50 @@ def measured_traffic(n_objects):
         return per_object * n_objects, f"profiles/ncu_cull_bake_traffic.json ({cap['objects']} objects, ncu --set full, kernel source {cap['kernel_source_sha16']}), scaled per object"
     except Exception as e:   # noqa: BLE001
         return None, f"unreadable capture: {e}"
+
+
+# --dump-outputs: at most 32 MB of visible list + 8 MB of matrices + 18 MB of frame samples, under 64 MB in all
+DUMP_VISIBLE_BYTES = 32 << 20
+DUMP_MATRIX_OBJECTS = 1 << 16
+DUMP_PIXELS = 1 << 19
+
+
+def seeded_sample(n, k, seed):
+    """Ascending positions of a fixed sample of k out of n (all n when n <= k), the same on every run."""
+    if n <= k:
+        return np.arange(n)
+    return np.sort(np.random.default_rng(seed).choice(n, k, replace=False))
+
+
+def dump_cull_bake(out_dir, backend, enabled):
+    """What a caller of the cull + bake step receives: the visible-object count, the ascending visible list (a fixed sample of its
+    positions past DUMP_VISIBLE_BYTES) and MV / MVP of a fixed sample of the enabled objects (disabled slots hold no defined matrices)."""
+    os.makedirs(out_dir, exist_ok=True)
+    n = len(enabled)
+    vis = backend.readback_visible(CAMERA_VIEWPORT)
+    id_type = np.float32 if n <= 1 << 24 else np.float64   # object ids stay exact
+    np.save(os.path.join(out_dir, "visible_count.npy"), np.array([len(vis)], dtype=np.float64))
+    np.save(os.path.join(out_dir, "visible_objects.npy"),
+            vis[seeded_sample(len(vis), DUMP_VISIBLE_BYTES // np.dtype(id_type).itemsize, 1)].astype(id_type))
+    ids = np.flatnonzero(enabled)
+    ids = ids[seeded_sample(len(ids), DUMP_MATRIX_OBJECTS, 2)]
+    chunk, parts = 1 << 20, []
+    for first in range(0, n, chunk):      # chunked so that the host copies stay small
+        sel = ids[(ids >= first) & (ids < first + chunk)]
+        if len(sel):
+            parts.append(backend.readback_object_matrices(CAMERA_VIEWPORT, first, int(sel[-1]) + 1 - first)[sel - first])
+    mats = np.concatenate(parts) if parts else np.zeros(0, dtype=OBJECT_MATRICES_DTYPE)
+    np.save(os.path.join(out_dir, "object_model_view.npy"), mats["model_view"].astype(np.float32))
+    np.save(os.path.join(out_dir, "object_model_view_proj.npy"), mats["model_view_proj"].astype(np.float32))
+
+
+def dump_frame(out_dir, backend):
+    """What a caller of the forward path receives, at a fixed sample of pixels: the tonemapped target, the HDR colour and the depth."""
+    os.makedirs(out_dir, exist_ok=True)
+    px = seeded_sample(backend.width * backend.height, DUMP_PIXELS, 3)
+    np.save(os.path.join(out_dir, "frame_ldr.npy"), backend.readback_ldr().reshape(-1, 4)[px].astype(np.float32))
+    np.save(os.path.join(out_dir, "frame_hdr.npy"), backend.readback_hdr_f16().reshape(-1, 4)[px].astype(np.float32))
+    np.save(os.path.join(out_dir, "frame_depth.npy"), backend.readback_depth().reshape(-1)[px].astype(np.float32))
 
 
 class ClockSampler:
@@ -255,6 +301,8 @@ def reference_arm(args):
     for _ in range(args.steps):
         b.object_uniform_upload(CAMERA_VIEWPORT, header, CB_BAKE | CB_CULL)
     dt = (time.perf_counter() - t0) / args.steps
+    if args.dump_outputs:
+        dump_cull_bake(args.dump_outputs, b, rec["enabled"])
     value = n / dt
     line = {
         "impl": "reference", "metric": METRIC, "value": value, "unit": "objects/s", "n_gpus": args.gpus, "steps": args.steps, "warmup": args.warmup,
@@ -304,7 +352,11 @@ def main():
     ap.add_argument("--no-forward", action="store_true")
     ap.add_argument("--no-dynamic", action="store_true")
     ap.add_argument("--forward-steps", type=int, default=5)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed (rank 0) as DIR/<name>.npy for comparing two builds")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl != "reference" else args.warmup
     if args.impl == "reference":
         return reference_arm(args)
@@ -422,6 +474,8 @@ def main():
     total_ms = max_over_ranks(starts[0].elapsed_time(final))
     launches = backend.launch_count() - launches0
     n_vis = backend.visible_count(CAMERA_VIEWPORT)
+    if args.dump_outputs and rank == 0:
+        dump_cull_bake(args.dump_outputs, backend, host_rec["enabled"])
     ms_per_step = total_ms / args.steps
     value = world * n / (ms_per_step * 1e-3)
     peak, peak_src = measured_peak_gbs()
@@ -632,6 +686,8 @@ def forward_section(args, torch, dist, load_cuda_backend, rank, world, local, de
     f1.record(fstream)
     barrier()
     frame_ms = max_over_ranks(f0.elapsed_time(f1) / args.forward_steps)
+    if args.dump_outputs and world == 1:   # with several ranks each one holds only its own rows of the frame
+        dump_frame(args.dump_outputs, fb)
     launches_per_frame = (fb.launch_count() - l0) // max(args.forward_steps, 1)
     st = torch.tensor([float(x) for x in fb.forward_stats()[:3]], device=dev, dtype=torch.float64)
     if world > 1:
