@@ -83,9 +83,12 @@ int r3_frame_graph_stats(r3_ctx* ctx, uint64_t stats[4]);
 /* optional per-stage device timing (off by default): when enabled, CUDA event pairs are recorded around the kernels below and
  * r3_stage_times returns, per stage, the summed duration in ms and the number of launches since the last call (it synchronises).
  * stage ids: 0 triangle_test_kernel, 1 raster_setup_kernel (colour passes), 2 raster_setup_kernel (shadow passes), 3 raster_band_kernel,
- * 4 resolve_kernel, 5 the batch_objects sort, 6 cull_bake_kernel, 7 triangle_compact_kernel. */
+ * 4 resolve_kernel, 5 the batch_objects sort, 6 cull_bake_kernel, 7 triangle_compact_kernel, 8 r3_generate_mipmaps (read with r3_stage_times_n). */
 int r3_set_stage_timing(r3_ctx* ctx, int enabled);
 int r3_stage_times(r3_ctx* ctx, double ms[8], uint32_t launches[8]);
+/* the same for the first n_stages stages (at most 9): stage 8 = r3_generate_mipmaps (mip_head / mip_level / mip_tail kernels of one call
+ * timed as one pair, launches = calls) */
+int r3_stage_times_n(r3_ctx* ctx, uint32_t n_stages, double* ms, uint32_t* launches);
 
 /* ------------------------------------------------------------------ world data
  * same bytes as the wgpu buffers named on the right */
@@ -108,6 +111,16 @@ int r3_set_textures(r3_ctx*, const r3_texture_desc* descs, uint32_t count, const
  * still holds its clear value.  desc->width = face size (height is ignored), six faces in the order +X, -X, +Y, -Y, +Z, -Z, each with
  * its `mip_count` levels stored tightly, face after face, from desc->byte_offset.  desc == NULL removes the skybox. */
 int r3_set_skybox(r3_ctx*, const r3_texture_desc* desc, const void* texels, uint64_t nbytes);
+/* MipmapGenerator::generate_mipmaps (rend3/src/util/mipmap.rs:139-219) for the textures TextureManager::add created with
+ * MipmapSource::Generated: levels 1 .. mip_count-1 of each listed table entry are computed from its level 0 by rule R12 and
+ * written into the resident texel blob.  The bytes of those levels that r3_set_textures uploaded are ignored.  Stream-ordered,
+ * no host synchronisation (capturable inside r3_frame_begin / r3_frame_end).  The whole list is validated first; R3_E_INVALID, with
+ * no byte changed, for an index outside the table or listed twice, mip_count > floor(log2(max(w, h))) + 1, two listed chains that
+ * overlap in the blob, or a format outside Rgba8Unorm(Srgb), Bgra8Unorm(Srgb), R8Unorm, Rg8Unorm, Rgb10a2Unorm, R16Float, Rg16Float,
+ * Rgba16Float (the formats wgpu guarantees FILTERABLE and RENDER_ATTACHMENT).  mip_count == 1 is a valid no-op. */
+int r3_generate_mipmaps(r3_ctx*, const uint32_t* texture_indices, uint32_t count);
+/* test / tool path: blocking copy of texel-blob bytes [byte_offset, byte_offset + nbytes) */
+int r3_readback_texels(r3_ctx*, uint64_t byte_offset, void* dst, uint64_t nbytes);
 int r3_set_directional_lights(r3_ctx*, const void* bytes, uint64_t nbytes,
                               uint32_t atlas_width, uint32_t atlas_height);         /* directional.rs:135-156 */
 int r3_set_point_lights(r3_ctx*, const void* bytes, uint64_t nbytes);              /* point.rs:58-74 */

@@ -57,6 +57,7 @@ struct EvalOutput {
     const void* mesh_buffer = nullptr; uint64_t mesh_bytes = 0;
     const r3_material* materials = nullptr; uint32_t n_materials = 0;
     const r3_texture_desc* textures = nullptr; uint32_t n_textures = 0; const void* texels = nullptr; uint64_t texel_bytes = 0;
+    const uint32_t* generated_textures = nullptr; uint32_t n_generated = 0;   // table entries added with MipmapSource::Generated (texture.rs:146-180)
     const r3_texture_desc* skybox = nullptr; const void* skybox_texels = nullptr; uint64_t skybox_bytes = 0;     // SkyboxRoutine's cube map (null = none)
     const void* directional_lights = nullptr; uint64_t directional_bytes = 0; uint32_t shadow_target_size[2] = {0, 0};
     const void* point_lights = nullptr; uint64_t point_bytes = 0;
@@ -92,6 +93,7 @@ public:
         if (ev.material_key) check(r3_set_object_sort_info(ctx_, ev.material_key, ev.sort_flags, ev.location, ev.n_slots));
         check(r3_set_mesh_buffer(ctx_, ev.mesh_buffer, ev.mesh_bytes));
         check(r3_set_textures(ctx_, ev.textures, ev.n_textures, ev.texels, ev.texel_bytes));
+        if (ev.n_generated) check(r3_generate_mipmaps(ctx_, ev.generated_textures, ev.n_generated));   // MipmapGenerator::generate_mipmaps
         check(r3_set_skybox(ctx_, ev.skybox, ev.skybox_texels, ev.skybox_bytes));
         check(r3_set_materials(ctx_, ev.materials, ev.n_materials));
         check(r3_set_directional_lights(ctx_, ev.directional_lights, ev.directional_bytes, ev.shadow_target_size[0], ev.shadow_target_size[1]));

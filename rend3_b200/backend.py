@@ -40,6 +40,7 @@ ENTRY_POINTS = [
     "readback_hiz", "forward_stats", "forward_light_evaluations", "device_ptr", "set_scissor_rows", "skin", "readback_mesh_buffer",
     "exchange_create", "exchange_connect", "exchange_words", "exchange_merge", "exchange_merged", "exchange_count", "exchange_counts", "exchange_destroy",
     "peer_create", "peer_connect", "peer_send_atlas_rect", "peer_send_rows", "peer_signal", "peer_wait", "peer_destroy", "clear_shadow_rect", "set_cull_shard",
+    "generate_mipmaps", "readback_texels", "stage_times_n",
 ]
 
 
@@ -119,6 +120,12 @@ class Backend:
         self._call("stage_times", ms, n)
         return {name: {"ms": float(ms[i]), "launches": int(n[i])} for i, name in enumerate(self.STAGES)}
 
+    def mipmap_stage_time(self):
+        """Stage 8 of the stage timer (r3_stage_times_n): r3_generate_mipmaps calls since the last read, ms summed over them."""
+        ms, n = (C.c_double * 9)(), (C.c_uint32 * 9)()
+        self._call("stage_times_n", C.c_uint32(9), ms, n)
+        return {"ms": float(ms[8]), "launches": int(n[8])}
+
     # ---- world data
     def set_objects(self, records: np.ndarray):
         records = np.ascontiguousarray(records)
@@ -154,6 +161,16 @@ class Backend:
         texels = np.ascontiguousarray(texels).view(np.uint8).reshape(-1)
         assert descs.dtype.itemsize == 32
         self._call("set_textures", _ptr(descs) if len(descs) else None, C.c_uint32(len(descs)), _ptr(texels) if len(texels) else None, C.c_uint64(len(texels)))
+
+    def generate_mipmaps(self, texture_indices):
+        """MipmapGenerator::generate_mipmaps for MipmapSource::Generated textures: levels 1.. of the listed table entries from level 0 (rule R12)."""
+        idx = np.ascontiguousarray(texture_indices, dtype=np.uint32).reshape(-1)
+        self._call("generate_mipmaps", _ptr(idx) if len(idx) else None, C.c_uint32(len(idx)))
+
+    def readback_texels(self, byte_offset: int, nbytes: int) -> np.ndarray:
+        out = np.zeros(nbytes, dtype=np.uint8)
+        self._call("readback_texels", C.c_uint64(byte_offset), _ptr(out) if nbytes else None, C.c_uint64(nbytes))
+        return out
 
     def set_skybox(self, desc: Optional[np.ndarray], texels: Optional[np.ndarray]):
         if desc is None:

@@ -39,7 +39,7 @@ struct r3_jobs {
 // optional per-stage device timing (r3_set_stage_timing / r3_stage_times): CUDA event pairs around the kernels named below, so that
 // bench.py can put a measured duration next to each kernel's algorithmic bytes / flops.  Off by default: no events are recorded.
 enum { R3_STAGE_TRIANGLE_TEST = 0, R3_STAGE_RASTER_SETUP_COLOUR, R3_STAGE_RASTER_SETUP_DEPTH, R3_STAGE_RASTER_BANDS, R3_STAGE_RESOLVE, R3_STAGE_SORT,
-       R3_STAGE_CULL_BAKE, R3_STAGE_TRIANGLE_COMPACT, R3_STAGE_COUNT };
+       R3_STAGE_CULL_BAKE, R3_STAGE_TRIANGLE_COMPACT, R3_STAGE_MIPMAPS, R3_STAGE_COUNT };
 struct r3_stage_timer {
     bool enabled = false;
     std::vector<cudaEvent_t> pool;            // recycled events: [2 k] start, [2 k + 1] stop
@@ -91,6 +91,15 @@ struct r3_camera {
     unsigned long long* d_block_sums = nullptr; uint64_t block_sums_cap = 0;
 };
 
+// one job of r3_generate_mipmaps' work list (r3_mipmap.cu): a texture's source level and how many levels one launch derives from it
+struct r3_mip_job {
+    uint64_t src_off;                         // byte offset of the source level in the texel blob
+    uint32_t sw, sh, fmt, levels;             // source size, format, levels produced (head: fused levels, level kernel: 1, tail: the rest)
+    uint32_t tiles_x;                         // head: 64x64 tiles per row; level kernel: 256-texel segments per destination row
+    uint32_t item_begin;                      // first work item of the job within its launch
+};
+static_assert(sizeof(r3_mip_job) == 32, "mip job");
+
 struct r3_tri_record { float xyw[3][3]; uint32_t object_id; uint32_t vid[3]; uint32_t _pad[3]; };   // 64 B
 static_assert(sizeof(r3_tri_record) == 64, "triangle record");
 
@@ -117,6 +126,12 @@ struct r3_ctx {
     r3_material* d_materials = nullptr; uint32_t n_materials = 0, materials_cap = 0;
     bool has_skybox = false; r3_texture_desc sky_desc{}; uint8_t* d_sky_texels = nullptr; uint64_t sky_cap = 0;   // cube map of the skybox routine
     r3_texture_desc* d_tex_descs = nullptr; uint32_t n_textures = 0, tex_descs_cap = 0; uint8_t* d_texels = nullptr; uint64_t texels_cap = 0;
+    std::vector<r3_texture_desc> tex_descs_host; uint64_t texel_bytes = 0;   // host copy of the table (r3_generate_mipmaps plans from it)
+    r3_mip_job* d_mip_jobs = nullptr; uint64_t mip_jobs_cap = 0; std::vector<uint8_t> mip_plan_host;   // work list of the last r3_generate_mipmaps
+    // pinned staging of work lists uploaded inside a recorded frame (the captured copy reads it when the graph runs): appended to, and
+    // rewound once the stream has drained (r3_stream_sync); a full arena is replaced by one twice as large and kept until the context goes
+    uint8_t* mip_staging = nullptr; uint64_t mip_staging_cap = 0, mip_staging_used = 0; std::vector<void*> mip_staging_retired;
+    bool mip_tail_smem_set = false;           // mip_tail_kernel's dynamic shared-memory limit raised
     r3_directional_light* d_dir = nullptr; uint32_t n_dir = 0, dir_cap = 0;
     r3_point_light* d_point = nullptr; uint32_t n_point = 0, point_cap = 0;
     float* d_light_mats = nullptr; uint64_t light_mats_cap = 0;   // view-space light tables built by light_prep_kernel
@@ -207,6 +222,7 @@ int r3_download_jobs(r3_ctx* c, r3_camera* cam);          // device-built jobs -
 int r3_compute_max_invocations(r3_ctx* c);
 void r3_new_frame_epoch(r3_ctx* c);          // the frame-wide sort of the previous frame is stale from here on
 int r3_blend_collect(r3_ctx* c, bool* ran);   // r3_raster.cu: per-sample fragment lists of the blend routine
+int r3_launch_mipmaps(r3_ctx* c, const uint32_t* indices, uint32_t count);   // r3_mipmap.cu: rule R12 over validated table indices
 int r3_iobuf_new(r3_ctx* c, r3_iobuf* b, uint64_t elems, uint64_t elem_size, bool clear_on_swap);
 int r3_iobuf_swap(r3_ctx* c, r3_iobuf* b, uint64_t new_elems);
 

@@ -1,5 +1,6 @@
 // r3_ctx.cu — context, uploads, readbacks and the C ABI glue of librend3_b200.so (include/rend3_b200.h).
 // Host logic only; the kernels live in r3_cull_bake.cu, r3_tri_cull.cu, r3_raster.cu, r3_shade.cu.
+#include <algorithm>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -75,6 +76,9 @@ R3_EXPORT int r3_ctx_destroy(r3_ctx* c) {
     r3_peer_destroy(c);
     if (!c->objects_borrowed) cudaFree(c->d_objects);
     cudaFree(c->d_hot_transform); cudaFree(c->d_hot_sphere); cudaFree(c->d_enabled_bits); cudaFree(c->d_tex_descs); cudaFree(c->d_texels); cudaFree(c->d_sky_texels);
+    cudaFree(c->d_mip_jobs);
+    if (c->mip_staging) cudaFreeHost(c->mip_staging);
+    for (void* p : c->mip_staging_retired) cudaFreeHost(p);
     cudaFree(c->d_sort_key8); cudaFree(c->d_sort_loc); cudaFree(c->d_gsort_keys[0]); cudaFree(c->d_gsort_keys[1]); cudaFree(c->d_gsort_hist); cudaFree(c->d_gsort_header);
     cudaFree(c->d_live_bits); cudaFree(c->d_mesh); cudaFree(c->d_materials); cudaFree(c->d_dir); cudaFree(c->d_point);
     cudaFree(c->d_light_mats); cudaFree(c->d_atlas);
@@ -164,9 +168,11 @@ cudaError_t r3_stream_sync(r3_ctx* c) {
         // was recorded, wait, and let the rest of the frame run eagerly
         const cudaError_t e = r3_submit_capture(c, -1);
         c->frames_flushed++;
-        if (e != cudaSuccess) return e;
+        if (e != cudaSuccess) { c->mip_plan_host.clear(); return e; }   // the recorded work-list copy never ran
     }
-    return cudaStreamSynchronize(c->stream);
+    const cudaError_t e = cudaStreamSynchronize(c->stream);
+    if (e == cudaSuccess) c->mip_staging_used = 0;   // every recorded copy out of the staging arena has run
+    return e;
 }
 R3_EXPORT int r3_frame_begin(r3_ctx* c) {
     if (!c) return R3_E_INVALID;
@@ -184,7 +190,10 @@ R3_EXPORT int r3_frame_end(r3_ctx* c) {
     const cudaError_t e = r3_submit_capture(c, (int)(c->frame_index & 1u));
     c->frame_index++;
     if (was) c->frames_graphed++;
-    if (e != cudaSuccess) return r3_cuda_fail(c, e, "frame_end (graph submission)");
+    if (e != cudaSuccess) {
+        c->mip_plan_host.clear();   // the recorded work-list copy never ran: the next r3_generate_mipmaps uploads its list again
+        return r3_cuda_fail(c, e, "frame_end (graph submission)");
+    }
     return R3_OK;
 }
 R3_EXPORT int r3_frame_graph_stats(r3_ctx* c, uint64_t stats[4]) {
@@ -218,19 +227,20 @@ R3_EXPORT int r3_set_stage_timing(r3_ctx* c, int enabled) {
     c->timer.used = 0;
     return R3_OK;
 }
-R3_EXPORT int r3_stage_times(r3_ctx* c, double ms[8], uint32_t launches[8]) {
-    if (!c || !ms || !launches) return R3_E_INVALID;
+R3_EXPORT int r3_stage_times_n(r3_ctx* c, uint32_t n_stages, double* ms, uint32_t* launches) {
+    if (!c || !ms || !launches || n_stages > R3_STAGE_COUNT) return r3_fail(c, R3_E_INVALID, "stage_times: bad arguments");
     cudaSetDevice(c->device);
     R3_CUDA(c, r3_stream_sync(c));
-    for (int k = 0; k < 8; ++k) { ms[k] = 0.0; launches[k] = 0; }
+    for (uint32_t k = 0; k < n_stages; ++k) { ms[k] = 0.0; launches[k] = 0; }
     r3_stage_timer& t = c->timer;
     for (size_t k = 0; k < t.used; ++k) {
         float e = 0.f;
-        if (cudaEventElapsedTime(&e, t.pool[2 * k], t.pool[2 * k + 1]) == cudaSuccess && t.stage_of[k] >= 0 && t.stage_of[k] < 8) { ms[t.stage_of[k]] += e; launches[t.stage_of[k]]++; }
+        if (cudaEventElapsedTime(&e, t.pool[2 * k], t.pool[2 * k + 1]) == cudaSuccess && t.stage_of[k] >= 0 && t.stage_of[k] < (int)n_stages) { ms[t.stage_of[k]] += e; launches[t.stage_of[k]]++; }
     }
     t.used = 0;
     return R3_OK;
 }
+R3_EXPORT int r3_stage_times(r3_ctx* c, double ms[8], uint32_t launches[8]) { return r3_stage_times_n(c, 8, ms, launches); }
 
 // ------------------------------------------------------------------ world data
 R3_EXPORT int r3_set_objects(r3_ctx* c, const r3_object* recs, uint32_t n) {
@@ -356,6 +366,46 @@ R3_EXPORT int r3_set_textures(r3_ctx* c, const r3_texture_desc* descs, uint32_t 
     if (nbytes) R3_CUDA(c, cudaMemcpyAsync(c->d_texels, texels, nbytes, cudaMemcpyHostToDevice, c->stream));
     R3_CUDA(c, r3_stream_sync(c));
     c->n_textures = n;
+    c->tex_descs_host.assign(descs, descs + n);
+    c->texel_bytes = nbytes;
+    return R3_OK;
+}
+// the formats wgpu guarantees FILTERABLE and RENDER_ATTACHMENT: what rend3-gltf asks MipmapSource::Generated for (rend3-gltf/src/lib.rs:1082-1087)
+static bool mip_format_ok(uint32_t f) {
+    return f == R3_TEXFMT_RGBA8_UNORM || f == R3_TEXFMT_RGBA8_UNORM_SRGB || f == R3_TEXFMT_BGRA8_UNORM || f == R3_TEXFMT_BGRA8_UNORM_SRGB || f == R3_TEXFMT_R8_UNORM ||
+           f == R3_TEXFMT_RG8_UNORM || f == R3_TEXFMT_RGB10A2_UNORM || f == R3_TEXFMT_R16_FLOAT || f == R3_TEXFMT_RG16_FLOAT || f == R3_TEXFMT_RGBA16_FLOAT;
+}
+R3_EXPORT int r3_generate_mipmaps(r3_ctx* c, const uint32_t* indices, uint32_t count) {
+    if (!c || (!indices && count)) return r3_fail(c, R3_E_INVALID, "generate_mipmaps: null");
+    // the whole list is checked before anything is launched: a rejected call changes no byte
+    std::vector<std::pair<uint64_t, uint64_t>> chains;
+    std::vector<uint8_t> seen(c->n_textures, 0);
+    for (uint32_t n = 0; n < count; ++n) {
+        const uint32_t i = indices[n];
+        if (i >= c->n_textures) return r3_fail(c, R3_E_INVALID, "generate_mipmaps: index outside the texture table");
+        if (seen[i]) return r3_fail(c, R3_E_INVALID, "generate_mipmaps: index listed twice");
+        seen[i] = 1;
+        const r3_texture_desc& d = c->tex_descs_host[i];
+        if (!mip_format_ok(d.format)) return r3_fail(c, R3_E_INVALID, "generate_mipmaps: format is not filterable and renderable");
+        uint32_t max_mips = 0;
+        for (uint32_t m = d.width > d.height ? d.width : d.height; m; m >>= 1) ++max_mips;   // floor(log2(max(w, h))) + 1
+        if (d.mip_count > max_mips) return r3_fail(c, R3_E_INVALID, "generate_mipmaps: mip_count exceeds floor(log2(max(w, h))) + 1");
+        uint64_t total = 0;
+        for (uint32_t l = 0; l < d.mip_count; ++l) total += R3_TEXFMT_LEVEL_BYTES(d.format, (d.width >> l) ? (d.width >> l) : 1u, (d.height >> l) ? (d.height >> l) : 1u);
+        chains.emplace_back(d.byte_offset, d.byte_offset + total);
+    }
+    std::sort(chains.begin(), chains.end());
+    for (size_t k = 1; k < chains.size(); ++k)
+        if (chains[k].first < chains[k - 1].second) return r3_fail(c, R3_E_INVALID, "generate_mipmaps: two listed mip chains overlap");
+    cudaSetDevice(c->device);
+    return r3_launch_mipmaps(c, indices, count);
+}
+R3_EXPORT int r3_readback_texels(r3_ctx* c, uint64_t byte_offset, void* dst, uint64_t nbytes) {
+    if (!c || (!dst && nbytes)) return r3_fail(c, R3_E_INVALID, "readback_texels: null");
+    if (byte_offset > c->texel_bytes || nbytes > c->texel_bytes - byte_offset) return r3_fail(c, R3_E_INVALID, "readback_texels: range outside the texel blob");
+    cudaSetDevice(c->device);
+    if (nbytes) R3_CUDA(c, cudaMemcpyAsync(dst, c->d_texels + byte_offset, nbytes, cudaMemcpyDeviceToHost, c->stream));
+    R3_CUDA(c, r3_stream_sync(c));
     return R3_OK;
 }
 R3_EXPORT int r3_set_skybox(r3_ctx* c, const r3_texture_desc* desc, const void* texels, uint64_t nbytes) {

@@ -58,6 +58,7 @@ int main(int argc, char** argv) {
         ev.materials = as<r3_material>(s, "materials", &n); ev.n_materials = (uint32_t)n;
         ev.textures = as<r3_texture_desc>(s, "tex_descs", &n); ev.n_textures = (uint32_t)n;
         ev.texels = as<uint8_t>(s, "texels", &n); ev.texel_bytes = n;
+        if (s.count("tex_generated")) { ev.generated_textures = as<uint32_t>(s, "tex_generated", &n); ev.n_generated = (uint32_t)n; }   // absent: none
         if (s.count("skybox_desc") && !s.at("skybox_desc").empty()) {
             ev.skybox = as<r3_texture_desc>(s, "skybox_desc");
             ev.skybox_texels = as<uint8_t>(s, "skybox_texels", &n); ev.skybox_bytes = n;

@@ -116,6 +116,8 @@ class BaseRenderGraph:
         b.set_object_sort_info(ev.object_material_key, flags.astype(np.uint8), loc)
         b.set_mesh_buffer(ev.mesh_buffer)
         b.set_textures(ev.texture_descs, ev.texture_texels)
+        if len(ev.generated_textures):                                            # TextureManager::add, MipmapSource::Generated (texture.rs:146-180)
+            b.generate_mipmaps(ev.generated_textures)
         b.set_skybox(ev.skybox_desc, ev.skybox_texels)
         b.set_materials(ev.material_buffer)
         b.set_directional_lights(ev.directional_buffer, ev.shadow_target_size[0], ev.shadow_target_size[1])

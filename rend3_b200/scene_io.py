@@ -33,6 +33,8 @@ def dump_scene(path: str, ev: EvalOutput, resolution: Tuple[int, int], samples: 
         _section(f, "materials", np.ascontiguousarray(ev.material_buffer).tobytes())
         _section(f, "tex_descs", np.ascontiguousarray(ev.texture_descs).tobytes())
         _section(f, "texels", np.ascontiguousarray(ev.texture_texels).tobytes())
+        if len(ev.generated_textures):   # older scene files have no such section: r3_frame reads it as empty
+            _section(f, "tex_generated", np.ascontiguousarray(ev.generated_textures, dtype=np.uint32).tobytes())
         _section(f, "skybox_desc", b"" if ev.skybox_desc is None else np.ascontiguousarray(ev.skybox_desc).tobytes())
         _section(f, "skybox_texels", b"" if ev.skybox_texels is None else np.ascontiguousarray(ev.skybox_texels).tobytes())
         _section(f, "dir_lights", bytes(ev.directional_buffer))

@@ -132,7 +132,7 @@ def subdivided_cube_mesh(k: int, with_uv: bool = False, vertex_alpha_seed: Optio
 
 
 def textured_cube_scene(n_objects: int = 300, seed: int = 41, resolution: Tuple[int, int] = (320, 180), texture_size: int = 32,
-                        sample_type: str = "linear", cutout: bool = False, block_compressed: bool = False) -> EvalOutput:
+                        sample_type: str = "linear", cutout: bool = False, block_compressed: bool = False, device_mips: bool = False) -> EvalOutput:
     """Cubes with texture coordinates and materials that exercise every texture slot and layout flag of PbrMaterial
     (opaque.wgsl:203-424): sRGB albedo, tri- and bi-component normal maps, combined / split AO-metallic-roughness, reflectance,
     clear coat, emissive, a scaled uv_transform0; one shadowed directional light and two point lights."""
@@ -194,6 +194,10 @@ def textured_cube_scene(n_objects: int = 300, seed: int = 41, resolution: Tuple[
             r.textures[handle].block_format = name
         if cutout:
             r.textures[alpha_tex].block_format = "bc3"
+    if device_mips:   # MipmapSource::Generated as rend3 does it: level 0 uploaded, the chain rendered on the device (r3_generate_mipmaps, rule R12)
+        for t in r.textures:
+            if t.mips == "generated" and t.block_format is None:
+                t.mips = "device"
     mat_ids = [r.add_material(m) for m in mats]
     r.set_camera_data(cube_example_camera(8.0))
     r.add_directional_light(DirectionalLight(color=(1, 1, 1), intensity=1.0, direction=(-1.0, -4.0, 2.0), distance=80.0, resolution=256))

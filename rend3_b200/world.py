@@ -191,7 +191,9 @@ def sphere_apply_transform(center, radius, m):
 @dataclass
 class Texture:
     """rend3_types::Texture (rend3-types/src/lib.rs:843-870): RGBA texels + MipmapSource.  `data` is (h, w, 4) uint8 (Rgba8Unorm /
-    Rgba8UnormSrgb) or float32 (Rgba32Float); mips = "generated" (box filter, MipmapCount::Maximum) or 1 level."""
+    Rgba8UnormSrgb) or float32 (Rgba32Float); mips = "generated" (box filter, MipmapCount::Maximum) or 1 level; mips = "device":
+    MipmapSource::Generated as rend3 does it — level 0 plus a zero-filled chain of MipmapCount::Maximum levels that r3_generate_mipmaps
+    fills on the device (rule R12)."""
 
     data: np.ndarray
     srgb: bool = False
@@ -246,13 +248,19 @@ class Texture:
         lv = self.levels()
         if self.storage is not None:
             from .texformats import pack
-            return [pack(self.storage, l) for l in lv]
-        if self.block_format is not None:
+            lv = [pack(self.storage, l) for l in lv]
+        elif self.block_format is not None:
             from .bc import encode
             if self.block_levels is not None:
                 return [np.ascontiguousarray(l, dtype=np.uint8).reshape(-1) for l in self.block_levels]
             return [encode(self.block_format, l) for l in lv]
-        return [np.ascontiguousarray(l[..., : self.channels]) for l in lv] if self.channels in (1, 2) and self.data.dtype == np.uint8 else lv
+        elif self.channels in (1, 2) and self.data.dtype == np.uint8:
+            lv = [np.ascontiguousarray(l[..., : self.channels]) for l in lv]
+        if self.mips == "device":
+            h, w = self.data.shape[:2]
+            bpp = np.ascontiguousarray(lv[0]).nbytes // (w * h)
+            lv = lv + [np.zeros(max(w >> l, 1) * max(h >> l, 1) * bpp, dtype=np.uint8) for l in range(1, max(w, h).bit_length())]
+        return lv
 
 
 @dataclass
@@ -535,6 +543,7 @@ class EvalOutput:
     camera: CameraState
     skybox_desc: Optional[np.ndarray] = None    # TEXTURE_DESC_DTYPE scalar (width = face size), None = no skybox
     skybox_texels: Optional[np.ndarray] = None  # six faces (+X -X +Y -Y +Z -Z), each with its mip chain
+    generated_textures: np.ndarray = field(default_factory=lambda: np.zeros(0, dtype=np.uint32))   # table indices of mips="device" textures
 
 
 class Renderer:
@@ -771,6 +780,7 @@ class Renderer:
             texture_texels=tex_blob,
             skybox_desc=sky_desc,
             skybox_texels=sky_blob,
+            generated_textures=np.array([i for i, t in enumerate(self.textures) if t.mips == "device"], dtype=np.uint32),
             directional_buffer=dbytes,
             point_buffer=pbytes,
             shadows=shadows,
